@@ -85,7 +85,9 @@ PER_TENSOR_SLACK = 4.0
 def assert_close(actual, expected, rtol=RTOL_FP32, atol_scale=1.0, what=""):
     """relative to the magnitude of the expected ARRAY (norm-wise): the right yardstick for fp32 sums whose individual
     elements may cancel to ~0.  When ``expected`` (or ``actual``) comes from flat_grads / flat_params the comparison runs
-    per parameter tensor, each normalised by its own max |expected|."""
+    per parameter tensor, each normalised by its own max |expected|.
+    Returns the measured error as a fraction of its bound (the larger of the norm-wise and the per-tensor ratio), so that a
+    caller can report the margin it passed with."""
     segments = getattr(expected, "segments", None) or getattr(actual, "segments", None)
     actual = np.asarray(actual, dtype=np.float64)
     expected = np.asarray(expected, dtype=np.float64)
@@ -93,12 +95,12 @@ def assert_close(actual, expected, rtol=RTOL_FP32, atol_scale=1.0, what=""):
     nan_a, nan_e = np.isnan(actual), np.isnan(expected)
     assert (nan_a == nan_e).all(), f"{what}: NaN pattern differs"
     if nan_e.all():
-        return
+        return 0.0
     gscale = max(np.abs(expected[~nan_e]).max(), 1e-30)
     err = np.abs(actual[~nan_e] - expected[~nan_e]).max() / gscale
     assert err <= rtol * atol_scale, f"{what}: max err / max|expected| = {err:.3e} > {rtol * atol_scale:.1e}"
     if segments is None or actual.ndim != 1:
-        return
+        return err / (rtol * atol_scale)
     worst = (0.0, "")
     for name, lo, hi in segments:
         a, e = actual[lo:hi], expected[lo:hi]
@@ -111,3 +113,4 @@ def assert_close(actual, expected, rtol=RTOL_FP32, atol_scale=1.0, what=""):
             worst = (err, name)
     bound = rtol * atol_scale * PER_TENSOR_SLACK
     assert worst[0] <= bound, f"{what}: tensor {worst[1]}: max err / max|expected tensor| = {worst[0]:.3e} > {bound:.1e}"
+    return max(err / (rtol * atol_scale), worst[0] / bound)

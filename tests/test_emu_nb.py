@@ -4,6 +4,7 @@ exercised by tests/test_gpu_nb.py."""
 import pytest
 
 from nb_cases import CASES, run_case
+import bf16_feature_cases as features
 
 
 @pytest.mark.parametrize("name", sorted(CASES))
@@ -18,3 +19,9 @@ def test_nb_batch_missing_mode(emu):
 @pytest.mark.parametrize("B", [1, 37, 129])
 def test_nb_tiny_and_ragged_batches(emu, B):
     run_case("dropout_mnar", "cpu", emu, B=B)
+
+
+@pytest.mark.parametrize("name", sorted(features.CASES))
+def test_nb_feature_case(emu, name):
+    """non-ReLU activations, 1- to 8-class decoders, mixed module kinds, permuted / partial sequences (tests/bf16_feature_cases.py)"""
+    features.run_feature_case(name, "cpu", emu, features.ENGINE_NB)

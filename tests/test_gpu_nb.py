@@ -12,6 +12,7 @@ from multimodn_b200 import MultiModNHistory, FusedAdam, _lib
 from helpers import flat_grads, assert_close
 from model_utils import model_from_spec, GradTap, tapped_flat
 from nb_cases import CASES, run_case, ENGINE_NB
+import bf16_feature_cases as features
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
@@ -20,6 +21,12 @@ DEV = "cuda"
 @pytest.mark.parametrize("name", sorted(CASES))
 def test_nb_case(name):
     run_case(name, DEV, _lib.get_lib())
+
+
+@pytest.mark.parametrize("name", sorted(features.CASES))
+def test_nb_feature_case(name):
+    """non-ReLU activations, 1- to 8-class decoders, mixed module kinds, permuted / partial sequences (tests/bf16_feature_cases.py)"""
+    features.run_feature_case(name, DEV, _lib.get_lib(), ENGINE_NB)
 
 
 def test_nb_batch_missing_mode():
